@@ -2,7 +2,7 @@
 """Benchmark of the level-synchronous DAG message-passing path (BASELINE.json metric:
 gates/s propagated fwd+bwd, all rounds, and train-step ms).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one training step of the reference's loop on one synthetic batch: Model.forward(G)
 (level schedule + struct encoder + level sweep), recon / prob / func losses, backward, gradient
@@ -10,7 +10,11 @@ all-reduce (N > 1) and Adam.  ``value`` = gates propagated per second over all r
 batches resident in HBM; ``e2e`` = the same through Trainer.train_step with the batch in pinned
 HOST memory (H2D copy and loss read-back inside the timed region).  ``--impl reference`` times the
 reference algorithm's CPU restatement (oracle/dg_oracle.py, per-node ``subgraph`` loop included)
-on the host cores -- the one other place this file executes oracle/.
+on the host cores -- the one other place this file executes oracle/.  ``--dump-outputs DIR`` writes
+what ``Trainer.train_step`` returned in the last timed step of ``value`` (losses, hs, hf, link
+predictions) as float32 ``DIR/<name>.npy``.  The same arguments give the same inputs in every run --
+the batches, the seeded weights (Adam runs at learning rate 0, see measure) and torch's seed for the
+step's random draws -- so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -27,6 +31,7 @@ for p in (os.path.join(ROOT, "multi-gate-vae_b200"), ROOT):
     if p not in sys.path:
         sys.path.insert(0, p)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 WORKLOADS = {
@@ -43,6 +48,26 @@ WORKLOADS = {
 }
 HANDLED = {"aig": (1, 2), "mig": (1, 2, 3, 4), "xmg": (1, 2, 3, 4, 5), "xag": (2, 3, 5)}
 LOSS_W = (1.0, 4.0, 4.0)      # stage-3 weights of the reference schedule (train.py:91)
+DUMP_BYTES = 60 * 10 ** 6     # --dump-outputs: data bytes of one dump, under 64 MB with the .npy headers
+
+
+def write_outputs(out_dir, arrays):
+    """``arrays`` (name -> CPU tensor) as float32 ``out_dir/<name>.npy``.  Above DUMP_BYTES in all, every array of more than one
+    row keeps the same share of its rows, drawn with a fixed seed (arrays of the same length keep the same rows), and
+    ``<name>_rows.npy`` (float64) lists the rows kept."""
+    os.makedirs(out_dir, exist_ok=True)
+    multi = {k for k, a in arrays.items() if a.dim() > 0 and a.shape[0] > 1}
+    fixed = sum(4 * a.numel() for k, a in arrays.items() if k not in multi)
+    per_share = sum(a.shape[0] * (4 * a[0].numel() + 8) for k, a in arrays.items() if k in multi)
+    share = min(1.0, (DUMP_BYTES - fixed) / max(per_share, 1))
+    for name, a in sorted(arrays.items()):
+        a = a.float()
+        if share < 1.0 and name in multi:
+            rows = torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:max(1, int(a.shape[0] * share))]
+            rows = rows.sort().values
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.double().numpy())
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def make_host_batch(w, rank, idx, own_sizes=False):
@@ -244,9 +269,11 @@ def _restore_stdout():
         _SAVED_STDOUT = None
 
 
-def measure(w, wname, steps, warmup, nb, dev, rank, world, clocks_index=None, cpu_baseline=False, own_sizes=False):
+def measure(w, wname, steps, warmup, nb, dev, rank, world, clocks_index=None, cpu_baseline=False, own_sizes=False,
+            dump_dir=None):
     """Times `steps` train steps of workload `w` (after the setup pass and `warmup` steps) device-resident and end to end.
-    Returns the record of this workload (the caller prints it, or nests it under "workloads")."""
+    Returns the record of this workload (the caller prints it, or nests it under "workloads").  `dump_dir`: where the
+    outputs of the last step of the device-resident timed region (the one `value` comes from) are written."""
     import deepgate
     from deepgate import _native, ops
     from oracle import dg_oracle as O   # only for cpu_baseline (rank 0, N == 1) and the seeded weights helper
@@ -260,8 +287,12 @@ def measure(w, wname, steps, warmup, nb, dev, rank, world, clocks_index=None, cp
     model.load_state_dict(sd, strict=False)                # same random-init weights on every rank
     tmp = tempfile.mkdtemp(prefix="mgv_bench_")
     import contextlib
+    # learning rate 0: the fused Adam kernel does all of its work (moments included) but leaves the weights at the seeded values,
+    # so every step starts from the same weights in every run.  With a rate > 0 the weights drift apart between runs: the
+    # backward's float atomics leave last-bit noise in the gradients, and Adam scales the gradients that are only noise (the
+    # biases in front of the readout's BatchNorm: mathematically zero) up to full steps.
     with contextlib.redirect_stdout(sys.stderr):          # the Trainer prints its device like the reference's: stdout carries ONE JSON line
-        trainer = deepgate.Trainer(None, model, training_id="bench", save_dir=tmp, lr=1e-4,
+        trainer = deepgate.Trainer(None, model, training_id="bench", save_dir=tmp, lr=0.0,
                                    rc_prob_func_weight=list(LOSS_W), device=str(dev), batch_size=w["batch"],
                                    distributed=False)
     if variational:
@@ -284,8 +315,14 @@ def measure(w, wname, steps, warmup, nb, dev, rank, world, clocks_index=None, cp
             torch.distributed.barrier()
             torch.cuda.synchronize(dev)
 
+    # only the step numbered keep["at"] holds on to its outputs: no step of a timed region runs with an earlier step's
+    # outputs still allocated
+    keep = {"at": -1}
+
     def step_resident(i):
         st = trainer.train_step(fresh(resident[i % nb]))
+        if i == keep["at"]:
+            keep["status"] = st
         return st["loss"]
 
     e2e_trace = [] if os.environ.get("MGV_BENCH_VERBOSE") else None
@@ -374,9 +411,13 @@ def measure(w, wname, steps, warmup, nb, dev, rank, world, clocks_index=None, cp
     if sampler:
         sampler.mark_begin()
     mallocs0 = torch.cuda.memory_stats(dev).get("num_device_alloc", 0)
+    keep["at"] = steps - 1 if dump_dir is not None else -1
     ms = timed(step_resident, steps)
+    keep["at"] = -1
     mallocs_resident = torch.cuda.memory_stats(dev).get("num_device_alloc", 0) - mallocs0
     launches = _native.lib().mgv_kernel_launches() - launches0
+    # copied to pageable host memory (no device allocation) before the next region; written after the last one
+    outputs = {k: v.detach().cpu() for k, v in keep.pop("status", {}).items() if torch.is_tensor(v)}
     # the same K steps once more with a CUDA-event pair around every library call (the per-kernel table and the roofline's launch
     # durations): ~30 event pairs per step cost the host ~0.1 ms, so they stay out of the region `value` is taken from; the
     # profiled region's own time is reported next to it (`profiled_ms_per_step`)
@@ -410,6 +451,8 @@ def measure(w, wname, steps, warmup, nb, dev, rank, world, clocks_index=None, cp
     from deepgate.schedule import check_deferred_errors
     check_deferred_errors()                   # asynchronous input validation of every schedule built above
     ops.set_precision("fp32")
+    if dump_dir is not None:
+        write_outputs(dump_dir, outputs)
 
     g_local = sum(gates_per_step[i % nb] for i in range(steps))
     g_all = torch.tensor([float(g_local)], device=dev, dtype=torch.float64)
@@ -544,10 +587,14 @@ def run_ours(args, w):
     dev = torch.device("cuda", local)
     if world > 1:
         torch.distributed.init_process_group("nccl", device_id=dev)
+    # the step's random draws (edge order, negative samples, dropout masks) are seeded from torch's seed: fixed, so that the same
+    # arguments give the same inputs in every run
+    torch.manual_seed(rank)
     # clocks are sampled by rank 0 only (its GPU): one nvidia-smi poller per rank makes 8 processes hammer the driver's locks and
     # the host cores during the timed region of an 8-rank run
     rec = measure(w, args.workload, args.steps, args.warmup, args.batches, dev, rank, world, clocks_index=local if rank == 0 else None,
-                  cpu_baseline=(rank == 0 and world == 1 and not args.no_cpu_baseline))
+                  cpu_baseline=(rank == 0 and world == 1 and not args.no_cpu_baseline),
+                  dump_dir=args.dump_outputs if rank == 0 else None)
     subs = {}
     if not args.no_sub_workloads and args.workload == "cfg2":
         for name, st, wu, nb in SUB_WORKLOADS:
@@ -582,7 +629,12 @@ def main():
     ap.add_argument("--batches", type=int, default=4, help="distinct synthetic batches rotated through the steps")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sub-workloads", action="store_true", help="skip the short cfg3 / cfg4 / cfg5 runs nested under 'workloads'")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl ours)")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     w = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, w)

@@ -1,26 +1,32 @@
 """Generate tests/golden/*.pt by executing the UNMODIFIED reference source
-(/root/reference/DG_VAE/deepgate) under the dependency shim in oracle/shim.
+(the DG_VAE directory of the reference checkout, package ``deepgate``) under the
+dependency shim in oracle/shim.
 
-TEST INFRASTRUCTURE.  Run in the build container only (the reference tree does not
-exist on the GPU box):
+TEST INFRASTRUCTURE.  Needs the reference checkout; the tests only read the files:
 
-    python oracle/make_golden.py            # writes tests/golden/<case>.pt
+    python oracle/make_golden.py <reference checkout>/DG_VAE    # writes tests/golden/<case>.pt
 
 Each file holds the inputs (synthetic circuits, seeds in SURVEY.md section 8d form),
 the weights (regenerable from ``oracle.dg_oracle.synth_state_dict(kind, seed)``, so
 only the seed is stored), and what the reference produced: forward_level (top_sort),
 the per-level / per-type incoming-edge lists (subgraph), hs, hf, the three losses
-and the gradient of ``1*recon + 4*prob + 4*func`` w.r.t. every parameter.
+and the gradient of ``1*recon + 4*prob + 4*func`` w.r.t. every parameter.  A gradient
+of more than GRAD_WHOLE entries is stored as a seeded sample of GRAD_SAMPLE of them
+(``sampled_grad``), which keeps every file under 1 MB.
 """
 import importlib.util
 import os
 import sys
+import zlib
 
 import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path[:0] = [os.path.join(ROOT, "oracle", "shim"), "/root/reference/DG_VAE", ROOT]
+if len(sys.argv) != 2:
+    sys.exit("usage: python oracle/make_golden.py <reference checkout>/DG_VAE")
+REFERENCE = os.path.abspath(sys.argv[1])
+sys.path[:0] = [os.path.join(ROOT, "oracle", "shim"), REFERENCE, ROOT]
 
 import deepgate                                              # noqa: E402  (the reference package)
 import deepgate.dg_ae_model_aig, deepgate.dg_ae_model_mig    # noqa: E402,E401
@@ -33,7 +39,7 @@ from torch_geometric.data import collate                     # noqa: E402  (shim
 
 from oracle.dg_oracle import GATE_MODULES, synth_state_dict  # noqa: E402
 
-assert deepgate.__file__.startswith("/root/reference/"), deepgate.__file__
+assert deepgate.__file__.startswith(REFERENCE + os.sep), deepgate.__file__
 _spec = importlib.util.spec_from_file_location(
     "mgv_synth", os.path.join(ROOT, "multi-gate-vae_b200", "deepgate", "synth.py"))
 synth = importlib.util.module_from_spec(_spec)
@@ -50,6 +56,19 @@ CASES = {
     "xag_b3_r1": ("xag", "xag", 3, 8, 120, 12, 1, 4, 14, False),
 }
 LOSS_W = (1.0, 4.0, 4.0)
+GRAD_WHOLE, GRAD_SAMPLE = 1024, 512
+
+
+def sampled_grad(name, t):
+    """``t`` itself up to GRAD_WHOLE entries; above, GRAD_SAMPLE entries drawn with a seed taken from the parameter
+    name, plus the largest |entry|, as {shape, index (flat, ascending), values, absmax} (tests/util.py reads both)."""
+    if t is None or t.numel() <= GRAD_WHOLE:
+        return t
+    flat = t.reshape(-1)
+    g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+    idx = torch.unique(torch.cat([torch.randperm(flat.numel(), generator=g)[:GRAD_SAMPLE], flat.abs().argmax().reshape(1)]))
+    return {"shape": tuple(t.shape), "index": idx.to(torch.int32), "values": flat[idx].clone(),
+            "absmax": flat.abs().max().clone()}
 
 
 def build_batch(kind, circuits):
@@ -124,7 +143,7 @@ def run_case(name):
     }
     if with_grads:
         total.backward()
-        out["grads"] = {k: (p.grad.detach().clone() if p.grad is not None else None)
+        out["grads"] = {k: sampled_grad(k, p.grad.detach().clone() if p.grad is not None else None)
                         for k, p in model.named_parameters()}
     return out
 

@@ -6,16 +6,13 @@ import pytest
 import torch
 
 from oracle import dg_oracle as O
+from util import absmax, rel
 
 CASES = ["mig_b4_r1", "aig_b4_r1", "xmg_b3_r2", "xag_b3_r1"]
 
 
 def load(golden_dir, name):
     return torch.load(os.path.join(golden_dir, name + ".pt"), weights_only=False)
-
-
-def rel(a, b):
-    return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
 
 
 def test_structural_kats(golden_dir):
@@ -78,7 +75,7 @@ def test_forward_and_losses_match_reference(golden_dir, name):
             if mathematically_zero:
                 # scale-relative bound (SURVEY.md section 7 hard part 3): pure rounding noise on both sides
                 kw = k.split(".")[0] + ".msg_k.weight"
-                assert float(got.abs().max()) <= 1e-4 * float(g["grads"][kw].abs().max()) + 1e-12, k
+                assert float(got.abs().max()) <= 1e-4 * absmax(g["grads"][kw]) + 1e-12, k
                 continue
             assert rel(got, ref) < 5e-5, (k, rel(got, ref))
 
