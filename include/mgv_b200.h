@@ -342,6 +342,44 @@ int mgv_linear_tc(const float* in, int64_t N, const float* W, const float* bias,
 
 int mgv_tc_selftest(int32_t mode, const float* A, const float* B, float* D, int32_t K, int32_t N, mgv_stream_t stream);
 
+/* ------------------------------------------------------------------ logic simulation (labels: signal probability, truth-table distance)
+ * Bit-parallel simulation of the batch under 64 input patterns per uint64 word, level by level over the schedule's
+ * (stream, level, code) lists (any `streams`).  What the reference's dataset tooling produces as `prob` and `tt_dis`.
+ *   fn_table_host int32 [MGV_NCODE], HOST: gate function of each code; MGV_FN_NONE marks a code the circuit kind lacks.
+ *     AIG: {INPUT, AND, NOT};  MIG / XMG / XAG (gate_to_index, parser.py:133): {INPUT, MAJ, NOT, AND, OR, XOR}.
+ *     AND, OR and XOR reduce over all predecessors (fan-in >= 2); NOT has fan-in 1, MAJ fan-in 3, INPUT fan-in 0.
+ *   code int32 [N] raw gate codes; level int32 [N] the schedule's levels.
+ * mgv_logic_sim_validate SYNCHRONISES and returns MGV_ERR_ARG naming the first bad node (undefined code, INPUT with
+ * predecessors, gate with fan-in 0, NOT / MAJ / AND / OR / XOR with the wrong fan-in, a predecessor not at a lower
+ * level), else the first pair with an id outside [0, N).  pairs int64 [2][P].  ws >= 16 bytes.  Run it before any pass:
+ * the pass assumes a valid circuit (and stays memory-safe, with meaningless counts, on an undefined code).
+ * mgv_logic_sim_pass simulates words [first_word, first_word + W) of every node:
+ *   mode MGV_SIM_RANDOM:     word w of an INPUT = mix(mix(seed) ^ (rank << 40 | w)), mix = the splitmix64 finaliser;
+ *   mode MGV_SIM_EXHAUSTIVE: pattern t = 64 w + bit, the INPUT takes bit `rank` of t;
+ *   input_rank int32 [N]: an INPUT's position among the INPUTs of its own circuit (other entries are not read);
+ *   sim: mgv_logic_sim_bytes(N, W) bytes, 32-byte aligned, scratch ([N][W rounded up to 4] words; INPUT words included);
+ *   ones uint64 [N] in/out: += patterns of the pass where node v is 1;
+ *   diff uint64 [P] in/out: += patterns of the pass where the two nodes of pair p differ (pairs / diff NULL when P = 0).
+ * Counts are integers, so the result is deterministic and independent of how the words are split into passes.
+ */
+#define MGV_FN_NONE 0
+#define MGV_FN_INPUT 1
+#define MGV_FN_AND 2
+#define MGV_FN_OR 3
+#define MGV_FN_XOR 4
+#define MGV_FN_NOT 5
+#define MGV_FN_MAJ 6
+#define MGV_SIM_RANDOM 0
+#define MGV_SIM_EXHAUSTIVE 1
+size_t mgv_logic_sim_bytes(int64_t N, int32_t W);
+int mgv_logic_sim_validate(const mgv_schedule* sch, const int32_t* code, const int32_t* level,
+                           const int32_t* fn_table_host, const int64_t* pairs, int64_t P,
+                           void* ws, size_t ws_bytes, mgv_stream_t stream);
+int mgv_logic_sim_pass(const mgv_schedule* sch, const int32_t* code, const int32_t* input_rank,
+                       const int32_t* fn_table_host, int32_t mode, uint64_t seed, int64_t first_word, int32_t W,
+                       uint64_t* sim, uint64_t* ones, const int64_t* pairs, int64_t P, uint64_t* diff,
+                       mgv_stream_t stream);
+
 #define MGV_OK 0
 #define MGV_ERR_ARG (-1)
 #define MGV_ERR_CUDA (-2)

@@ -89,6 +89,10 @@ _PROTOTYPES = {
     "mgv_linear_wgrad": (ctypes.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
     "mgv_linear_tc": (ctypes.c_int, [_vp, _i64, _vp, _vp, _i32, _i32, _i32, _vp, _vp]),
     "mgv_tc_selftest": (ctypes.c_int, [_i32, _vp, _vp, _vp, _i32, _i32, _vp]),
+    "mgv_logic_sim_bytes": (_sz, [_i64, _i32]),
+    "mgv_logic_sim_validate": (ctypes.c_int, [_SP, _vp, _vp, ctypes.POINTER(_i32), _vp, _i64, _vp, _sz, _vp]),
+    "mgv_logic_sim_pass": (ctypes.c_int, [_SP, _vp, _vp, ctypes.POINTER(_i32), _i32, ctypes.c_uint64, _i64, _i32,
+                                          _vp, _vp, _vp, _i64, _vp, _vp]),
 }
 EXPORTED_SYMBOLS = tuple(_PROTOTYPES)
 
