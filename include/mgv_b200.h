@@ -199,25 +199,24 @@ int mgv_level_sweep_bwd(const mgv_schedule* sch, int32_t rounds, uint32_t handle
  *      0 Wcx[192][76]  cols 0..63 = Wc, cols 64..64+feat-1 = weight_ih_l0[:, 64:], rest 0
  *  14592 Whh[192][68]  weight_hh_l0, cols 64..67 = 0
  *  27648 bc[192]   27840 bih[192]   28032 bhh[192]   28224 ln_w[64]   28288 ln_b[64]   (pad to 28416)
- * x: float [N][feat] (feat <= MGV_MAX_FEAT).  states: float [num_enc][2*rounds+1][N][64] out
- * (slot 0 = ones, written by the call; slot 2*rounds = encoder output).
+ * x: float [N][feat] (feat <= MGV_MAX_FEAT).  states: float [num_enc][2][N][64] out, ping-pong slots: step k reads
+ * slot (k-1)&1 and writes slot k&1 (slot 0 starts as ones, written by the call; after the last step it holds the encoder output).
  * tiles: NULL (inference) or mgv_struct_tiles_bytes(N, num_enc, rounds) bytes out: the [agg | h | x deg 1] tensor-core operand
  * tile of every step ([num_enc][2*rounds][ceil(N/128)][73728 bytes], fp16 hi/lo planes), which mgv_struct_encoder_bwd
- * recomputes from instead of gathering the neighbour sums a second time (precision MGV_PRECISION_FP32 only).
+ * recomputes from instead of gathering the neighbour sums a second time.
  */
 size_t mgv_struct_fwd_workspace_bytes(int64_t N, int32_t num_enc);
 size_t mgv_struct_tiles_bytes(int64_t N, int32_t num_enc, int32_t rounds);
 int mgv_struct_encoder_fwd(const mgv_schedule* sch, int32_t num_enc, int32_t rounds, int32_t layernorm,
                            int32_t feat, const float* x, const float* weights, float* states, void* tiles,
                            void* ws, size_t ws_bytes, int32_t precision, mgv_stream_t stream);
-/* gout: float [num_enc][N][64] = d loss / d (encoder output).  grads: float
- * [num_enc][2][MGV_STRUCT_GRAD_FLOATS] out, SAME layout as the weight block (d Wcx, d Whh, d bc, d bih, d bhh,
- * d ln_w, d ln_b; padding columns are zero).  The host maps d Wc / d bc back to msg.* and weight_ih_l0. */
-int mgv_struct_bwd_grid(void);
+/* tiles: the operand tiles mgv_struct_encoder_fwd saved (required).  gout: float [num_enc][N][64] = d loss / d (encoder
+ * output).  grads: float [num_enc][2][MGV_STRUCT_GRAD_FLOATS] out, SAME layout as the weight block (d Wcx, d Whh, d bc,
+ * d bih, d bhh, d ln_w, d ln_b; padding columns are zero).  The host maps d Wc / d bc back to msg.* and weight_ih_l0. */
 size_t mgv_struct_bwd_workspace_bytes(int64_t N, int32_t num_enc);
 int mgv_struct_encoder_bwd(const mgv_schedule* sch, int32_t num_enc, int32_t rounds, int32_t layernorm,
-                           int32_t feat, const float* x, const float* weights, const float* states,
-                           const void* tiles, const float* gout, float* grads, void* ws, size_t ws_bytes,
+                           int32_t feat, const float* x, const float* weights, const void* tiles,
+                           const float* gout, float* grads, void* ws, size_t ws_bytes,
                            int32_t precision, mgv_stream_t stream);
 
 /* ------------------------------------------------------------------ fused reparam + KL + func loss

@@ -201,14 +201,6 @@ __device__ __forceinline__ float pow2_scale(float amax) {
     return __uint_as_float((uint32_t)(k + 127) << 23);
 }
 
-// Keep the running scale while amax * cur stays inside [2^2, 2^13] (fp16 tops out at 2^16): rescaling the
-// persistent weight-gradient fragments is then rare.
-__device__ __forceinline__ float pow2_scale_keep(float amax, float cur) {
-    const float v = amax * cur;
-    if (v >= 4.0f && v <= 8192.0f) return cur;
-    return (amax > 0.f) ? pow2_scale(amax) : cur;
-}
-
 __device__ __forceinline__ float pow2_scale_band(float amax, float cur, float lo, float hi) {
     const float v = amax * cur;
     if (v >= lo && v <= hi) return cur;

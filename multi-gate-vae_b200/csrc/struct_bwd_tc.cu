@@ -21,18 +21,11 @@
 // recompute (256) + data-gradient (128) + weight-gradient (288) columns, hence the split; the hand-off buffers are
 // processed in chunks of tiles so they stay L2-sized.
 #include <stdlib.h>
-#include <string.h>
 #include "struct_layout.cuh"
 
 long long* mgv_debug_trace();
 size_t mgv_struct_image_bytes(int num_enc);
 int mgv_struct_build_image(const float* weights, int num_enc, uint8_t* image, int precision, cudaStream_t st);
-int mgv_struct_bwd_legacy_grid(void);
-size_t mgv_struct_bwd_legacy_workspace_bytes(int64_t N, int32_t num_enc);
-int mgv_struct_encoder_bwd_legacy(const mgv_schedule* sch, int32_t num_enc, int32_t rounds, int32_t layernorm,
-                                  int32_t feat, const float* x, const float* weights, const float* states,
-                                  const float* gout, float* grads, void* ws, size_t ws_bytes, int32_t precision,
-                                  mgv_stream_t stream);
 
 namespace {
 using namespace struct_layout;
@@ -863,13 +856,9 @@ int chunk_tiles() {
     return v > 0 ? v : CHUNK_TILES_DEFAULT;
 }
 
-bool use_legacy(int precision) {
-    (void)precision;                    // both precisions run the tcgen05 kernels (bf16: single-plane instantiations)
-    const char* e = getenv("MGV_STRUCT_BWD");
-    return e && !strcmp(e, "mma");
-}
+}  // namespace
 
-size_t tc_workspace_bytes(int64_t N, int num_enc) {
+extern "C" size_t mgv_struct_bwd_workspace_bytes(int64_t N, int32_t num_enc) {
     int sms = 148;
     sm_count(&sms);
     const int64_t ntiles = (N + TM - 1) / TM;
@@ -885,22 +874,10 @@ size_t tc_workspace_bytes(int64_t N, int num_enc) {
     return b;
 }
 
-}  // namespace
-
-extern "C" int mgv_struct_bwd_grid(void) { return mgv_struct_bwd_legacy_grid(); }
-
-extern "C" size_t mgv_struct_bwd_workspace_bytes(int64_t N, int32_t num_enc) {
-    const size_t a = mgv_struct_bwd_legacy_workspace_bytes(N, num_enc), b = tc_workspace_bytes(N, num_enc);
-    return a > b ? a : b;
-}
-
 extern "C" int mgv_struct_encoder_bwd(const mgv_schedule* sch, int32_t num_enc, int32_t rounds, int32_t layernorm,
-                                      int32_t feat, const float* x, const float* weights, const float* states,
-                                      const void* tiles, const float* gout, float* grads, void* ws, size_t ws_bytes,
+                                      int32_t feat, const float* x, const float* weights, const void* tiles,
+                                      const float* gout, float* grads, void* ws, size_t ws_bytes,
                                       int32_t precision, mgv_stream_t stream) {
-    if (use_legacy(precision))
-        return mgv_struct_encoder_bwd_legacy(sch, num_enc, rounds, layernorm, feat, x, weights, states, gout, grads, ws, ws_bytes,
-                                             precision, stream);
     cudaStream_t st = (cudaStream_t)stream;
     MGV_REQUIRE(sch != nullptr, "struct encoder: null schedule");
     MGV_REQUIRE(num_enc >= 1 && num_enc <= 2, "struct encoder: num_enc must be 1 or 2");
@@ -926,7 +903,6 @@ extern "C" int mgv_struct_encoder_bwd(const mgv_schedule* sch, int32_t num_enc, 
     const int gxp = sms / num_enc > 0 ? sms / num_enc : 1;
     const int steps = 2 * rounds;
     const size_t slot = (size_t)N * D;
-    (void)states;          // the tcgen05 path recomputes from the saved operand tiles; only the mma.sync path reads the states
 
     MgvArena a(ws, ws_bytes);
     uint8_t* image = a.take<uint8_t>((size_t)num_enc * 2 * IMG_BYTES);

@@ -12,7 +12,7 @@
 // memory; biases and the degree term ride along as two extra K columns, so the epilogue is gates + LayerNorm.
 //
 // Persistent CTAs (one per SM, weights resident in shared memory for the whole launch), warp-specialised
-// (default shape: 8 epilogue + 16 gather + 1 MMA warp; the kernel is templated on it):
+// (8 epilogue + 16 gather + 1 MMA warp; the kernel is templated on the split):
 //   gather      neighbour sums, own state and [x deg 1] -> fp16 hi/lo -> operand tile (UMMA layout), 2 rows per lane;
 //               rows come in descending-degree order (mgv_build_degree_order) so a warp's lanes run equal trip counts;
 //               in a training step the same chunks also go to the tile image in HBM that the backward recomputes from
@@ -20,7 +20,6 @@
 //   epilogue    two threads per node = TMEM lane (32 units each): tensor memory -> GRU gates -> LayerNorm -> state_k
 //               (two accumulator buffers: the epilogue of tile t overlaps the gather and MMAs of tile t+1)
 #include <stdlib.h>
-#include <string.h>
 #include "struct_layout.cuh"
 
 namespace {
@@ -477,14 +476,9 @@ extern "C" int mgv_struct_encoder_fwd(const mgv_schedule* sch, int32_t num_enc, 
     if (rc != MGV_OK) return rc;
     const int steps = 2 * rounds;
     const size_t slot = (size_t)N * D;
-    const size_t enc_stride = (size_t)(steps + 1) * slot;
-    // launch shape: 16 gather warps x 2 rows per lane + 8 epilogue warps (25 warps, 72 registers), or the 13-warp shape
-    // (8 gather warps x 4 rows, 4 epilogue warps, 128 registers) with MGV_STRUCT_FWD=v1 (A/B)
-    const char* fwd_env = getenv("MGV_STRUCT_FWD");
-    const bool wide = !(fwd_env && !strcmp(fwd_env, "v1"));
-    MGV_CUDA(cudaFuncSetAttribute((const void*)struct_fwd_tc_kernel<false, 4, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)F_SMEM));
+    const size_t enc_stride = 2 * slot;
+    // launch shape: 16 gather warps x 2 rows per lane + 8 epilogue warps (25 warps, 72 registers)
     MGV_CUDA(cudaFuncSetAttribute((const void*)struct_fwd_tc_kernel<false, 2, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)F_SMEM));
-    MGV_CUDA(cudaFuncSetAttribute((const void*)struct_fwd_tc_kernel<true, 4, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)F_SMEM));
     MGV_CUDA(cudaFuncSetAttribute((const void*)struct_fwd_tc_kernel<true, 2, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)F_SMEM));
     int dev = 0, sms = 0;
     MGV_CUDA(cudaGetDevice(&dev));
@@ -510,17 +504,15 @@ extern "C" int mgv_struct_encoder_fwd(const mgv_schedule* sch, int32_t num_enc, 
         p.tile_cost = dir == 0 ? sch->tile_cost_in : sch->tile_cost_out;
         p.x = x;
         p.image = image + (size_t)dir * IMG_BYTES;
-        p.prev = states + (size_t)(k - 1) * slot;
-        p.next = states + (size_t)k * slot;
+        p.prev = states + (size_t)((k - 1) & 1) * slot;      // two slots, ping-pong: the last step (2 * rounds) writes slot 0
+        p.next = states + (size_t)(k & 1) * slot;
         p.enc_stride = enc_stride;
         // tile buffer [enc][step][tile][A_TILE_BYTES] (fp16 hi/lo planes; bf16 mode writes its single bf16 plane into the hi slots)
         p.tiles = tiles ? (uint8_t*)tiles + (size_t)(k - 1) * ntiles * A_TILE_BYTES : nullptr;
         p.tiles_enc_stride = (size_t)steps * ntiles * A_TILE_BYTES;
         p.trace = (k == trace_step) ? g_trace : nullptr;
-        if (precision == 1 && wide) struct_fwd_tc_kernel<true, 2, 8><<<dim3(gx, num_enc), 25 * 32, F_SMEM, st>>>(p);
-        else if (precision == 1) struct_fwd_tc_kernel<true, 4, 4><<<dim3(gx, num_enc), 13 * 32, F_SMEM, st>>>(p);
-        else if (wide) struct_fwd_tc_kernel<false, 2, 8><<<dim3(gx, num_enc), 25 * 32, F_SMEM, st>>>(p);
-        else struct_fwd_tc_kernel<false, 4, 4><<<dim3(gx, num_enc), 13 * 32, F_SMEM, st>>>(p);
+        if (precision == 1) struct_fwd_tc_kernel<true, 2, 8><<<dim3(gx, num_enc), 25 * 32, F_SMEM, st>>>(p);
+        else struct_fwd_tc_kernel<false, 2, 8><<<dim3(gx, num_enc), 25 * 32, F_SMEM, st>>>(p);
         mgv_count_launches(1);
     }
     return mgv_check_cuda(cudaGetLastError(), "mgv_struct_encoder_fwd");

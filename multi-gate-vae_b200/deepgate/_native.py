@@ -64,9 +64,8 @@ _PROTOTYPES = {
     "mgv_struct_fwd_workspace_bytes": (_sz, [_i64, _i32]),
     "mgv_struct_tiles_bytes": (_sz, [_i64, _i32, _i32]),
     "mgv_struct_encoder_fwd": (ctypes.c_int, [_SP, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
-    "mgv_struct_bwd_grid": (ctypes.c_int, []),
     "mgv_struct_bwd_workspace_bytes": (_sz, [_i64, _i32]),
-    "mgv_struct_encoder_bwd": (ctypes.c_int, [_SP, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
+    "mgv_struct_encoder_bwd": (ctypes.c_int, [_SP, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _i32, _vp]),
     "mgv_vae_func_workspace_bytes": (_sz, [_i64]),
     "mgv_vae_func_loss_fwd": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "mgv_vae_func_loss_bwd": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _i64,

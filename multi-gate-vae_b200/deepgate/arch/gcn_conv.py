@@ -1,5 +1,5 @@
 """AggConv parameter holder (reference arch/gcn_conv.py:15-45): msg_i = sum_{j->i} (W h_j + b).
-The arithmetic runs inside the fused struct-encoder step kernel (csrc/struct_encoder.cu)."""
+The arithmetic runs inside the fused struct-encoder step kernels (csrc/struct_tc.cu, csrc/struct_bwd_tc.cu)."""
 import torch.nn as nn
 
 

@@ -2,7 +2,7 @@
 
 ``MultiGCNEncoder`` / ``DirectMultiGCNEncoder`` keep the reference's constructor arguments,
 sub-module names (aggr, update, aggr_r, update_r, ln -> checkpoint keys) and forward signatures;
-the computation is the fused CUDA step kernel of csrc/struct_encoder.cu.
+the computation runs in the fused CUDA step kernels of csrc/struct_tc.cu (forward) and csrc/struct_bwd_tc.cu (backward).
 """
 import torch
 import torch.nn as nn

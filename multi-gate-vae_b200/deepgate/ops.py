@@ -293,7 +293,7 @@ class StructEncoderFunction(torch.autograd.Function):
         enc_params = [params[e * per:(e + 1) * per] for e in range(num_enc)]
         prec = _prec()
         pack = _struct_pack(enc_params, layernorm, dev)
-        states = torch.empty(num_enc, 2 * rounds + 1, max(N, 1), nat.D, dtype=torch.float32, device=dev)
+        states = torch.empty(num_enc, 2, max(N, 1), nat.D, dtype=torch.float32, device=dev)     # ping-pong slots
         # training: the forward also saves every step's tensor-core operand tile; the backward recomputes from those
         # instead of gathering the neighbour sums a second time (bf16 mode: the single bf16 plane of each tile)
         need_tiles = N > 0 and any(ctx.needs_input_grad[5:])
@@ -310,16 +310,16 @@ class StructEncoderFunction(torch.autograd.Function):
         ctx.tiles = tiles
         ctx.csr, ctx.rounds, ctx.layernorm, ctx.num_enc, ctx.feat, ctx.per = csr, rounds, layernorm, num_enc, feat, per
         ctx.prec = prec
-        ctx.save_for_backward(x_c, pack, states)
+        ctx.save_for_backward(x_c, pack)
         ctx.saved_params = params
-        # one output per encoder (views of the last state slot): indexing a stacked [num_enc, N, 64] output costs the backward two
-        # zero-fills, two slice copies and an add of N x 64 tensors (autograd's select backward), 50 us at cfg2
-        return tuple(states[e, 2 * rounds, :N] for e in range(num_enc))
+        # one output per encoder (views of slot 0, which the last step writes): indexing a stacked [num_enc, N, 64] output costs
+        # the backward two zero-fills, two slice copies and an add of N x 64 tensors (autograd's select backward), 50 us at cfg2
+        return tuple(states[e, 0, :N] for e in range(num_enc))
 
     @staticmethod
     def backward(ctx, *gouts):
         lib = nat.lib()
-        x_c, pack, states = ctx.saved_tensors
+        x_c, pack = ctx.saved_tensors
         csr, rounds, num_enc, feat, per = ctx.csr, ctx.rounds, ctx.num_enc, ctx.feat, ctx.per
         dev = x_c.device
         N, D = csr.N, nat.D
@@ -338,7 +338,7 @@ class StructEncoderFunction(torch.autograd.Function):
             ws = nat.workspace(nb, dev)
             with _timed("struct_encoder_bwd", dev):
               nat.check(lib.mgv_struct_encoder_bwd(csr.c_struct(), num_enc, rounds, int(ctx.layernorm), feat,
-                                                 nat.ptr(x_c), nat.ptr(pack), nat.ptr(states), nat.ptr(ctx.tiles), nat.ptr(g),
+                                                 nat.ptr(x_c), nat.ptr(pack), nat.ptr(ctx.tiles), nat.ptr(g),
                                                  nat.ptr(grads), nat.ptr(ws), nb, ctx.prec, nat.stream_of(dev)),
                       "mgv_struct_encoder_bwd")
         params = ctx.saved_params

@@ -155,6 +155,68 @@ def multi_gcn_encoder(P, name, x6, ei, rounds, layernorm):
     return state
 
 
+class _RoundGrad(torch.autograd.Function):
+    """Identity whose backward rounds the incoming gradient to ``dtype``."""
+
+    @staticmethod
+    def forward(ctx, v, dtype):
+        ctx.dtype = dtype
+        return v.view_as(v)
+
+    @staticmethod
+    def backward(ctx, g):
+        return g.to(ctx.dtype).to(g.dtype), None
+
+
+def multi_gcn_encoder_composed(P, name, x6, ei, rounds, layernorm, round=None):
+    """``multi_gcn_encoder`` written the way the struct-encoder kernels compute a step: the GRU pre-activations are one
+    product of the tile [sum of neighbour states | h | x | deg | 1] with the AggConv linear composed into the GRU input
+    weights (Wc = W_ih[:, :64] W_msg, bc = W_ih[:, :64] b_msg, csrc/pack.cu) and the r / z biases merged.  With
+    ``round`` (e.g. torch.bfloat16) every tile operand and weight entry is rounded to that type in the forward
+    (straight-through) and the four gate pre-activation gradients (r, z, gi_n, gh_n) are rounded to it in the backward,
+    as the low-precision kernels do; everything else stays in the parameters' type."""
+    dim = P[name + ".aggr.msg.weight"].size(0)
+    dt = P[name + ".aggr.msg.weight"].dtype
+    state = torch.ones(x6.size(0), dim, dtype=dt)
+    x6 = x6.to(dt)
+    ones = torch.ones(x6.size(0), 1, dtype=dt)
+
+    def rnd(v):
+        return v if round is None else v + (v.to(round).to(dt) - v).detach()
+
+    def rnd_grad(v):
+        return v if round is None else _RoundGrad.apply(v, round)
+
+    def ln(v):
+        return F.layer_norm(v, (dim,), P[name + ".ln.weight"], P[name + ".ln.bias"], 1e-5) if layernorm else v
+
+    def step(mod, agg_mod, h, e):
+        w_msg, b_msg = P[agg_mod + ".msg.weight"], P[agg_mod + ".msg.bias"]
+        w_ih, w_hh = P[mod + ".weight_ih_l0"], P[mod + ".weight_hh_l0"]
+        b_ih, b_hh = P[mod + ".bias_ih_l0"], P[mod + ".bias_hh_l0"]
+        agg = torch.zeros_like(h).index_add(0, e[1], h.index_select(0, e[0]))
+        deg = torch.zeros(h.size(0), 1, dtype=dt).index_add(0, e[1], torch.ones(e.size(1), 1, dtype=dt))
+        tile = torch.cat([agg, h, x6, deg, ones], 1)
+        # weights over the tile columns agg | h | x | deg of gi = W_ih [msg || x] (msg = W_msg agg + deg b_msg) and gh = W_hh h
+        g3, nx = 3 * dim, x6.size(1) + 1
+        w_gi = torch.cat([w_ih[:, :dim] @ w_msg, torch.zeros(g3, dim, dtype=dt), w_ih[:, dim:], (w_ih[:, :dim] @ b_msg)[:, None]], 1)
+        w_gh = torch.cat([torch.zeros(g3, dim, dtype=dt), w_hh, torch.zeros(g3, nx, dtype=dt)], 1)
+        # accumulator columns r | z | gi_n | gh_n; the last tile column carries the biases
+        w = torch.cat([w_gi[:2 * dim] + w_gh[:2 * dim], w_gi[2 * dim:], w_gh[2 * dim:]], 0)
+        b = torch.cat([b_ih[:2 * dim] + b_hh[:2 * dim], b_ih[2 * dim:], b_hh[2 * dim:]])
+        pre = rnd(tile) @ rnd(torch.cat([w, b[:, None]], 1)).t()
+        r_pre, z_pre, gi_n, gh_n = (rnd_grad(v) for v in pre.split(dim, 1))
+        r, z = torch.sigmoid(r_pre), torch.sigmoid(z_pre)
+        n = torch.tanh(gi_n + r * gh_n)
+        return ln((1.0 - z) * n + z * h)
+
+    rei = torch.stack([ei[1], ei[0]], dim=0)
+    for _ in range(rounds):
+        state = step(name + ".update", name + ".aggr", state, ei)
+        state = step(name + ".update_r", name + ".aggr_r", state, rei)
+    return state
+
+
 def struct_encoder(P, enc, code, ei, s_rounds, t_rounds, layernorm):
     """DirectMultiGCNEncoder.forward (digae_layer.py:294-297) on the feature the
     models really feed it: one_hot(G.x[:,1], 6) where G.x is already one-hot, i.e.

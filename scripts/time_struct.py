@@ -17,5 +17,5 @@ def run(n):
     return tf / n, tb / n
 run(3)
 f, b = run(10)
-print("N=%d E=%d  struct fwd %.3f ms  bwd %.3f ms  (chunk=%s, path=%s)" % (G.x.size(0), G.edge_index.size(1), f, b,
-      os.environ.get("MGV_STRUCT_CHUNK", "default"), os.environ.get("MGV_STRUCT_BWD", "tcgen05")))
+print("N=%d E=%d  struct fwd %.3f ms  bwd %.3f ms  (chunk=%s)" % (G.x.size(0), G.edge_index.size(1), f, b,
+      os.environ.get("MGV_STRUCT_CHUNK", "default")))

@@ -20,15 +20,7 @@ lib.mgv_debug_set_trace(ctypes.c_void_p(tr.data_ptr()))
 torch.cuda.synchronize()
 lib.mgv_debug_set_trace(ctypes.c_void_p(0))
 t = tr.view(2 * 74, 16, 16).cpu().double()
-if os.environ.get("MGV_STRUCT_BWD") == "mma":
-    names = ["gather", "step GEMM + gates", "LN backward", "GRU bwd + amax + DG store", "data-grad GEMMs + stores", "weight-grad GEMMs", "end barrier"]
-    valid = (t[:, :, 0] > 0) & (t[:, :, 7] > 0)
-    for i, n in enumerate(names):
-        d = (t[:, :, i + 1] - t[:, :, i])[valid]
-        print("%-28s mean %7.0f  med %7.0f  max %7.0f cycles" % (n, d.mean(), d.median(), d.max()))
-    d = (t[:, :, 7] - t[:, :, 0])[valid]
-    print("tile total mean %.0f cycles" % d.mean())
-elif os.environ.get("MGV_TRACE_WGRAD"):
+if os.environ.get("MGV_TRACE_WGRAD"):
     spans = [("producer: wait stage empty", 0, 1), ("stage: copies issued -> landed", 1, 2), ("rescale + hand-over", 2, 3),
              ("MMA: wait ready", 4, 5), ("MMA: issue", 5, 6)]
     valid = (t[:, :, 0] > 0) & (t[:, :, 6] > 0)

@@ -80,6 +80,33 @@ def test_forward_and_losses_match_reference(golden_dir, name):
             assert rel(got, ref) < 5e-5, (k, rel(got, ref))
 
 
+def test_composed_struct_encoder_equals_the_encoder():
+    """The kernel-shaped restatement (one tile product per step, AggConv composed into the GRU input weights) is the same
+    function as multi_gcn_encoder: outputs and every parameter gradient agree in float64."""
+    g = torch.Generator().manual_seed(12)
+    n = 90
+    src, dst = [], []
+    for i in range(1, n):                       # random DAG: up to 3 distinct predecessors among 0 .. i-1
+        for j in torch.randperm(i, generator=g)[:min(i, int(torch.randint(1, 4, (1,), generator=g)))].tolist():
+            src.append(j); dst.append(i)
+    ei = torch.tensor([src, dst])
+    x6 = torch.nn.functional.one_hot(torch.randint(0, 2, (n,), generator=g), 6)
+    w = torch.randn(n, 64, generator=g, dtype=torch.float64)
+    name = "mig_struct_encoder.source_conv"
+    out = []
+    for fn in (O.multi_gcn_encoder, O.multi_gcn_encoder_composed):
+        P = {k: v.clone().requires_grad_(True) for k, v in O.synth_state_dict("mig", 45, dtype=torch.float64).items()
+             if k.startswith(name + ".")}
+        s = fn(P, name, x6, ei, 2, True)
+        (s * w).sum().backward()
+        out.append((s.detach(), {k: p.grad for k, p in P.items()}))
+    (s0, g0), (s1, g1) = out
+    assert rel(s1, s0) < 1e-12
+    assert g0.keys() == g1.keys() and len(g0) == 14
+    for k in g0:
+        assert rel(g1[k], g0[k]) < 1e-12, (k, rel(g1[k], g0[k]))
+
+
 def test_vae_matches_reference(golden_dir):
     v = load(golden_dir, "vae")
     s, t = v["s"].clone().requires_grad_(True), v["t"].clone().requires_grad_(True)
