@@ -379,6 +379,36 @@ int mgv_logic_sim_pass(const mgv_schedule* sch, const int32_t* code, const int32
                        uint64_t* sim, uint64_t* ones, const int64_t* pairs, int64_t P, uint64_t* diff,
                        mgv_stream_t stream);
 
+/* ------------------------------------------------------------------ equivalence classes from simulation words
+ * Nodes equal on every simulated pattern, or complementary (one's words the bitwise NOT of the other's) on every one,
+ * share a class; exhaustive mode makes this exact functional equivalence, random mode equality on the simulated patterns.
+ * `sim` is the scratch of mgv_logic_sim_pass for the same N and W (row pitch W rounded up to 4 words), read after it.
+ * mgv_sim_signature_pass, once after each simulation pass (words [first_word, first_word + W)):
+ *   h0 / h1 uint64 [N] in/out (zero before the first pass): += mix(mix(g) ^ word) / mix(mix(g) ^ ~word) over the pass's
+ *   words, g = the word's global index, mix = the splitmix64 finaliser, sums mod 2^64 (independent of the pass split);
+ *   bit0 uint8 [N] out: written by the pass with first_word = 0, the node's value on pattern 0.
+ * mgv_sim_classes_group: key = mix(circuit ^ (bit0 ? h1 : h0)), stable radix sort of (key, node id); a run of equal keys is
+ *   a class, its smallest node id the representative.  circuit int32 [N]: the circuit of each node (nodes of different
+ *   circuits never share a class).  rep int64 [N] out: the representative; complemented uint8 [N] out: 1 when the node
+ *   computes the complement of its representative.  ws: mgv_sim_classes_bytes(N) bytes.
+ * mgv_sim_classes_verify_pass, once after each simulation pass (any pass split): checks a class assignment (rep,
+ *   complemented) word by word and sets bad[v] = 1 (bad uint8 [N] in/out, zero before the first pass) when v is a member
+ *   whose words are not equal (complemented 0) or complementary (complemented 1) to its representative's, whose
+ *   representative lies in another circuit, outside [0, N) or is not its own representative, or when v is a
+ *   representative with complemented != 0.
+ * mgv_sim_classes_split SYNCHRONISES: every node with bad[v] != 0 becomes a singleton (rep[v] = v, complemented[v] = 0);
+ *   *n_split_host = how many.  ws >= 8 bytes.
+ */
+int mgv_sim_signature_pass(const uint64_t* sim, int64_t N, int32_t W, int64_t first_word, uint64_t* h0, uint64_t* h1,
+                           uint8_t* bit0, mgv_stream_t stream);
+size_t mgv_sim_classes_bytes(int64_t N);
+int mgv_sim_classes_group(const uint64_t* h0, const uint64_t* h1, const uint8_t* bit0, const int32_t* circuit, int64_t N,
+                          int64_t* rep, uint8_t* complemented, void* ws, size_t ws_bytes, mgv_stream_t stream);
+int mgv_sim_classes_verify_pass(const uint64_t* sim, int64_t N, int32_t W, const int32_t* circuit, const int64_t* rep,
+                                const uint8_t* complemented, uint8_t* bad, mgv_stream_t stream);
+int mgv_sim_classes_split(int64_t N, int64_t* rep, uint8_t* complemented, const uint8_t* bad, void* ws, size_t ws_bytes,
+                          int64_t* n_split_host, mgv_stream_t stream);
+
 #define MGV_OK 0
 #define MGV_ERR_ARG (-1)
 #define MGV_ERR_CUDA (-2)

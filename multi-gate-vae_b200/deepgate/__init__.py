@@ -16,6 +16,6 @@ from . import parser, parser_func, parser_func_others
 from .parser import NpzParser, CircuitDataset, read_npz_file
 from .parser_func_others import parse_pyg_mlpgate, circuits_to_batch
 from .utils import dag_utils
-from .simulate import simulate, simulate_counts, label_circuits, write_npz
+from .simulate import simulate, simulate_counts, equivalence_classes, label_circuits, write_npz
 from .utils.utils import zero_normalization, AverageMeter
 from .__version__ import __version__
