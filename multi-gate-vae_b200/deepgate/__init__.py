@@ -17,5 +17,6 @@ from .parser import NpzParser, CircuitDataset, read_npz_file
 from .parser_func_others import parse_pyg_mlpgate, circuits_to_batch
 from .utils import dag_utils
 from .simulate import simulate, simulate_counts, equivalence_classes, label_circuits, write_npz
+from .aiger import read_aiger, read_aiger_files
 from .utils.utils import zero_normalization, AverageMeter
 from .__version__ import __version__

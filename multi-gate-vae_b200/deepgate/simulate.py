@@ -6,6 +6,7 @@ under random inputs) and the truth-table distance of node pairs (``tt_sim`` in a
     write_npz(labelled, "graphs.npz", "labels.npz", "mig")  # the reference's on-disk layouts, read back by NpzParser
     rep, complemented, n_split = equivalence_classes(G, "mig")   # functionally equal / complementary gates
     python -m deepgate.simulate --graphs graphs.npz --type mig --out DIR [--class-pairs K]
+    python -m deepgate.simulate --aiger FILE_OR_DIR ... --type mig --out DIR  # AIGER netlists (deepgate/aiger.py)
 
 Gate functions by code: AIG {0 INPUT, 1 AND, 2 NOT}; MIG / XMG / XAG {0 INPUT, 1 MAJ, 2 NOT, 3 AND, 4 OR, 5 XOR}.  AND, OR
 and XOR reduce over all their predecessors, NOT takes one, MAJ three.  Random mode: ``patterns`` (a multiple of 64) patterns;
@@ -345,9 +346,13 @@ def read_circuits(graphs_path, kind):
 
 def main(argv=None):
     ap = argparse.ArgumentParser(prog="python -m deepgate.simulate",
-                                 description="Label the circuits of a graphs.npz by logic simulation on cuda:0 and write "
-                                             "DIR/graphs.npz (+ DIR/labels.npz for mig / xmg / xag), readable by NpzParser.")
-    ap.add_argument("--graphs", required=True, help="input graphs.npz (the reference layout of --type)")
+                                 description="Label the circuits of a graphs.npz or of AIGER files by logic simulation on "
+                                             "cuda:0 and write DIR/graphs.npz (+ DIR/labels.npz for mig / xmg / xag), "
+                                             "readable by NpzParser.")
+    src = ap.add_mutually_exclusive_group(required=True)
+    src.add_argument("--graphs", help="input graphs.npz (the reference layout of --type)")
+    src.add_argument("--aiger", nargs="+", metavar="FILE_OR_DIR",
+                     help="input AIGER netlists: .aag / .aig files, or directories of them (deepgate/aiger.py)")
     ap.add_argument("--type", required=True, choices=sorted(CODE_TABLES))
     ap.add_argument("--out", required=True, help="output directory")
     ap.add_argument("--patterns", type=int, default=32768, help="random patterns, a multiple of 64")
@@ -359,7 +364,14 @@ def main(argv=None):
     args = ap.parse_args(argv)
     if not 0 <= args.class_pairs <= args.pairs:
         ap.error("--class-pairs must be in [0, --pairs]")
-    circuits = read_circuits(args.graphs, args.type)
+    if args.aiger:
+        from .aiger import read_aiger_files
+        circuits = read_aiger_files(args.aiger, args.type)
+        dropped = sum(int((c["outputs"] < 0).sum()) for c in circuits)
+        if dropped:
+            print("dropped %d outputs that fold to constants" % dropped)
+    else:
+        circuits = read_circuits(args.graphs, args.type)
     labelled = label_circuits(circuits, args.type, "cuda:0", n_pairs=args.pairs, class_pairs=args.class_pairs,
                               patterns=args.patterns, seed=args.seed, exhaustive=args.exhaustive)
     os.makedirs(args.out, exist_ok=True)
