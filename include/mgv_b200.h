@@ -409,6 +409,29 @@ int mgv_sim_classes_verify_pass(const uint64_t* sim, int64_t N, int32_t W, const
 int mgv_sim_classes_split(int64_t N, int64_t* rep, uint8_t* complemented, const uint8_t* bad, void* ws, size_t ws_bytes,
                           int64_t* n_split_host, mgv_stream_t stream);
 
+/* ------------------------------------------------------------------ mapping (AIG -> single MIG / XMG / XAG gates)
+ * csrc/map_cuts.cu has the exact definitions (cuts of at most 3 leaves with 8-bit truth tables, support reduction,
+ * dominance, aliases, area-flow ranking in saturating uint32, 16 kept cuts per node).  The batch is an AIG (codes INPUT 0,
+ * AND 1, NOT 2; ANDs of fan-in 2, NOTs of fan-in 1, checked by the caller); `sch` its level schedule with streams = 1.
+ *   levels_host int32 [n_levels][2], HOST: (first position in sch->order, count) of the AND nodes of each level that has
+ *   some, in level order; one launch per entry (mgv_map_cover walks them in reverse).
+ *   match int32 [256]: per truth table, gate | input-complement mask << 3 | output complement << 6, or -1 (no gate).
+ * mgv_map_cuts: per node, best int32 [N][4] (best cut leaves, -1 padded; table | leaves << 8), best_match int32 [N]
+ *   (match entry of the best cut, -1 for INPUTs, NOTs and aliases), flow uint32 [N] (area flow of the best cut) and alias
+ *   int32 [N] (-3: not an alias; else the node's literal 2 u + complemented, -2 / -1 the constants).  ws:
+ *   mgv_map_cuts_bytes(N) bytes (kept cuts, fan-outs).
+ * mgv_map_cover: required uint8 [N] out: 1 for the non-NOT nodes of the roots (roots int32 [n_roots], any node ids,
+ *   resolved through NOTs and aliases; constants mark nothing) and, from the last level down, for the leaves of the best
+ *   cut of every required AND that is not an alias.
+ */
+size_t mgv_map_cuts_bytes(int64_t N);
+int mgv_map_cuts(const mgv_schedule* sch, const int32_t* code, const int32_t* match, const int32_t* levels_host,
+                 int32_t n_levels, int32_t* best, int32_t* best_match, uint32_t* flow, int32_t* alias, void* ws,
+                 size_t ws_bytes, mgv_stream_t stream);
+int mgv_map_cover(const mgv_schedule* sch, const int32_t* code, const int32_t* roots, int64_t n_roots,
+                  const int32_t* levels_host, int32_t n_levels, const int32_t* best, const int32_t* alias,
+                  uint8_t* required, mgv_stream_t stream);
+
 #define MGV_OK 0
 #define MGV_ERR_ARG (-1)
 #define MGV_ERR_CUDA (-2)

@@ -8,7 +8,7 @@ NVCC="${NVCC:-/usr/local/cuda/bin/nvcc}"
 FLAGS=(-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -Xcompiler -O2 ${MGV_NVCC_EXTRA:-})
 OBJS=()
 pids=()
-for f in mgv_error schedule sweep sweep_tc struct_tc struct_bwd_tc linear linear_tc vae_func recon readout pack tc_selftest logic_sim sim_classes; do
+for f in mgv_error schedule sweep sweep_tc struct_tc struct_bwd_tc linear linear_tc vae_func recon readout pack tc_selftest logic_sim sim_classes map_cuts; do
   "${NVCC}" "${FLAGS[@]}" -c "${HERE}/${f}.cu" -o "${OUT}/${f}.o" &
   pids+=($!)
   OBJS+=("${OUT}/${f}.o")

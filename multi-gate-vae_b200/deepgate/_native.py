@@ -97,6 +97,9 @@ _PROTOTYPES = {
     "mgv_sim_classes_group": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _sz, _vp]),
     "mgv_sim_classes_verify_pass": (ctypes.c_int, [_vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp]),
     "mgv_sim_classes_split": (ctypes.c_int, [_i64, _vp, _vp, _vp, _vp, _sz, ctypes.POINTER(_i64), _vp]),
+    "mgv_map_cuts_bytes": (_sz, [_i64]),
+    "mgv_map_cuts": (ctypes.c_int, [_SP, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "mgv_map_cover": (ctypes.c_int, [_SP, _vp, _vp, _i64, _vp, _i32, _vp, _vp, _vp, _vp]),
 }
 EXPORTED_SYMBOLS = tuple(_PROTOTYPES)
 

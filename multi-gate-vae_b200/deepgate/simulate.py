@@ -7,6 +7,7 @@ under random inputs) and the truth-table distance of node pairs (``tt_sim`` in a
     rep, complemented, n_split = equivalence_classes(G, "mig")   # functionally equal / complementary gates
     python -m deepgate.simulate --graphs graphs.npz --type mig --out DIR [--class-pairs K]
     python -m deepgate.simulate --aiger FILE_OR_DIR ... --type mig --out DIR  # AIGER netlists (deepgate/aiger.py)
+    python -m deepgate.simulate --aiger FILE_OR_DIR ... --type xmg --map --out DIR  # mapped onto XMG gates first
 
 Gate functions by code: AIG {0 INPUT, 1 AND, 2 NOT}; MIG / XMG / XAG {0 INPUT, 1 MAJ, 2 NOT, 3 AND, 4 OR, 5 XOR}.  AND, OR
 and XOR reduce over all their predecessors, NOT takes one, MAJ three.  Random mode: ``patterns`` (a multiple of 64) patterns;
@@ -361,15 +362,27 @@ def main(argv=None):
     ap.add_argument("--pairs", type=int, default=64, help="node pairs drawn per circuit that has none")
     ap.add_argument("--class-pairs", type=int, default=0,
                     help="of those, up to this many drawn among functionally equivalent or complementary nodes")
+    ap.add_argument("--map", action="store_true",
+                    help="with --aiger and --type mig / xmg / xag: read the files as AIGs and map them onto the gates of "
+                         "--type on cuda:0 first (deepgate/mapping.py)")
     args = ap.parse_args(argv)
     if not 0 <= args.class_pairs <= args.pairs:
         ap.error("--class-pairs must be in [0, --pairs]")
+    if args.map and (args.graphs or args.type == "aig"):
+        ap.error("--map takes --aiger input and --type mig, xmg or xag")
     if args.aiger:
         from .aiger import read_aiger_files
-        circuits = read_aiger_files(args.aiger, args.type)
+        circuits = read_aiger_files(args.aiger, "aig" if args.map else args.type)
         dropped = sum(int((c["outputs"] < 0).sum()) for c in circuits)
         if dropped:
             print("dropped %d outputs that fold to constants" % dropped)
+        if args.map:
+            from .mapping import gate_counts, map_circuits
+            ands = sum(int((c["x"][:, 1] == 1).sum()) for c in circuits)
+            circuits = map_circuits(circuits, args.type, "cuda:0")
+            counts = gate_counts(circuits, args.type)
+            print("mapped %d circuits: %d ANDs in; out %s" % (len(circuits), ands, ", ".join(
+                "%d %s" % (counts[g], g) for g in CODE_TABLES[args.type] if g != "INPUT")))
     else:
         circuits = read_circuits(args.graphs, args.type)
     labelled = label_circuits(circuits, args.type, "cuda:0", n_pairs=args.pairs, class_pairs=args.class_pairs,
