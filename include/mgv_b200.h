@@ -379,6 +379,35 @@ int mgv_logic_sim_pass(const mgv_schedule* sch, const int32_t* code, const int32
                        uint64_t* sim, uint64_t* ones, const int64_t* pairs, int64_t P, uint64_t* diff,
                        mgv_stream_t stream);
 
+/* ------------------------------------------------------------------ sequential simulation (labels of netlists with latches)
+ * Each of the 64 bits of a word is one trace of the circuit from its reset state; words [first_word, first_word + W) of
+ * the T trace words are simulated for `cycles` clock cycles in one launch (same gate functions and fn_table_host as
+ * above; random INPUT words only).
+ *   latches int64 [n_latch][3]: the latch's INPUT node; its next-state literal 2 u + complemented over the nodes (-2 / -1
+ *   the constants 0 / 1; another latch or the latch itself allowed); its reset: 0, 1, or 2 = uninitialised.
+ *   Trace word w starts with latch state 0, ~0, or (uninitialised) mix(mix(seed) ^ (rank << 40 | w)), rank = the latch
+ *   INPUT's input_rank.  Cycle t: every other INPUT takes mix(mix(seed) ^ (rank << 40 | (t T + w))), every node is
+ *   evaluated from the INPUTs and the state s_t, then s_{t+1} = the words of the next-state literals.
+ *   ones uint64 [N] in/out: += ones of node v over cycles t in [warmup, cycles) and the pass's traces (a latch INPUT counts
+ *   the state it holds in cycle t); diff uint64 [P] in/out likewise for the two nodes of pair p differing.
+ * mgv_seq_sim_validate SYNCHRONISES and returns MGV_ERR_ARG naming the first bad latch: node outside [0, N), node not an
+ *   INPUT, node of two latches, next-state node outside [0, N) or in another circuit (circuit int32 [N]), reset not in
+ *   {0, 1, 2}; or cycles < 1, warmup outside [0, cycles).  ws >= 8 + 4 N bytes.  Run it, and mgv_logic_sim_validate,
+ *   before any pass.
+ * mgv_seq_sim_pass: cycles x T <= MGV_SEQ_MAX_WORDS (word indices stay below the rank bits); ws = mgv_seq_sim_bytes(N,
+ *   n_latch, W) bytes, 32-byte aligned, scratch.  Counts are integers, independent of the split of the T trace words
+ *   into passes.
+ */
+#define MGV_SEQ_MAX_WORDS 1099511627776
+size_t mgv_seq_sim_bytes(int64_t N, int32_t n_latch, int32_t W);
+int mgv_seq_sim_validate(const mgv_schedule* sch, const int32_t* code, const int32_t* fn_table_host, const int32_t* circuit,
+                         const int64_t* latches, int32_t n_latch, int32_t cycles, int32_t warmup, void* ws,
+                         size_t ws_bytes, mgv_stream_t stream);
+int mgv_seq_sim_pass(const mgv_schedule* sch, const int32_t* code, const int32_t* input_rank, const int32_t* fn_table_host,
+                     const int64_t* latches, int32_t n_latch, uint64_t seed, int64_t first_word, int32_t W, int64_t T,
+                     int32_t cycles, int32_t warmup, void* ws, size_t ws_bytes, uint64_t* ones, const int64_t* pairs,
+                     int64_t P, uint64_t* diff, mgv_stream_t stream);
+
 /* ------------------------------------------------------------------ equivalence classes from simulation words
  * Nodes equal on every simulated pattern, or complementary (one's words the bitwise NOT of the other's) on every one,
  * share a class; exhaustive mode makes this exact functional equivalence, random mode equality on the simulated patterns.

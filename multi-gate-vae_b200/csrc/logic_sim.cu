@@ -7,6 +7,13 @@
 // wait that could hang.  One thread per node of the current level: load SIM_S words of each predecessor (one sector each),
 // apply the gate function, store SIM_S words, and add the node's ones to ones[v] (integer atomics).
 // Predecessor words are written earlier in the same kernel, so they are read with plain loads (never the non-coherent path).
+//
+// Sequential simulation (seq_sim_kernel): each of the 64 bits of a word is one trace of the circuit from its reset state.
+// CTA b runs every clock cycle of the traces of its slice in one launch: per cycle the level walk above (primary INPUTs
+// take the word of index t * T + trace word, latch INPUTs copy their state row), then every latch's next-state word is
+// staged into its state row and read back by the next cycle's walk, with a __syncthreads() between -- so latch-to-latch
+// chains and self-loops read the old state.  Each counted cycle adds one 64-bit atomic per node and per pair per slice,
+// as logic_sim_kernel does: measured faster than 32-bit counters per (slice, node) reduced after the pass (DESIGN.md §4.7).
 #include "mgv_common.cuh"
 
 namespace {
@@ -55,6 +62,40 @@ __device__ __forceinline__ void load4(const uint64_t* p, uint64_t (&v)[SIM_S]) {
     v[0] = lo.x; v[1] = lo.y; v[2] = hi.x; v[3] = hi.y;
 }
 
+// Words [w0, w0 + SIM_S) of gate v with function fn (not INPUT, not NONE) from its predecessors' words: the one copy of
+// the gate semantics, shared by logic_sim_kernel and seq_sim_kernel.
+__device__ __forceinline__ void gate_words(const SimArgs& a, int v, int fn, int w0, uint64_t (&out)[SIM_S]) {
+    const int p0 = a.in_ptr[v], p1 = a.in_ptr[v + 1];
+    load4(a.sim + (size_t)a.in_src[p0] * a.ld + w0, out);
+    if (fn == MGV_FN_NOT) {
+#pragma unroll
+        for (int k = 0; k < SIM_S; ++k) out[k] = ~out[k];
+    } else if (fn == MGV_FN_MAJ) {
+        uint64_t b[SIM_S], d[SIM_S];
+        load4(a.sim + (size_t)a.in_src[p0 + 1] * a.ld + w0, b);
+        load4(a.sim + (size_t)a.in_src[p0 + 2] * a.ld + w0, d);
+#pragma unroll
+        for (int k = 0; k < SIM_S; ++k) out[k] = (out[k] & b[k]) | (out[k] & d[k]) | (b[k] & d[k]);
+    } else {
+        for (int q = p0 + 1; q < p1; ++q) {
+            uint64_t b[SIM_S];
+            load4(a.sim + (size_t)a.in_src[q] * a.ld + w0, b);
+#pragma unroll
+            for (int k = 0; k < SIM_S; ++k)
+                out[k] = fn == MGV_FN_AND ? (out[k] & b[k]) : fn == MGV_FN_OR ? (out[k] | b[k]) : (out[k] ^ b[k]);
+        }
+    }
+}
+
+__device__ __forceinline__ void store4(uint64_t* p, const uint64_t (&v)[SIM_S]) {
+    reinterpret_cast<ulonglong2*>(p)[0] = make_ulonglong2(v[0], v[1]);
+    reinterpret_cast<ulonglong2*>(p)[1] = make_ulonglong2(v[2], v[3]);
+}
+
+__device__ __forceinline__ int node_fn(const SimArgs& a, int c) {
+    return (c >= 0 && c < MGV_NCODE) ? (int)((a.fn_bits >> (4 * c)) & 15u) : MGV_FN_NONE;
+}
+
 __global__ void __launch_bounds__(SIM_THREADS) logic_sim_kernel(const SimArgs a) {
     const int w0 = blockIdx.x * SIM_S;
     const int nw = min(SIM_S, a.W - w0);            // valid words of this slice (the last CTA may hold a partial one)
@@ -64,38 +105,16 @@ __global__ void __launch_bounds__(SIM_THREADS) logic_sim_kernel(const SimArgs a)
             const int beg = a.seg_ptr[seg], end = a.seg_ptr[seg + MGV_NCODE];
             for (int t = beg + threadIdx.x; t < end; t += blockDim.x) {
                 const int v = a.order[t];
-                const int c = a.code[v];
-                const int fn = (c >= 0 && c < MGV_NCODE) ? (int)((a.fn_bits >> (4 * c)) & 15u) : MGV_FN_NONE;     // validated before any pass
+                const int fn = node_fn(a, a.code[v]);       // validated before any pass
                 uint64_t out[SIM_S] = {0, 0, 0, 0};
                 if (fn == MGV_FN_INPUT) {
                     const int r = a.rank[v];
 #pragma unroll
                     for (int k = 0; k < SIM_S; ++k) out[k] = input_word(a, r, a.first_word + w0 + k);
                 } else if (fn != MGV_FN_NONE) {
-                    const int p0 = a.in_ptr[v], p1 = a.in_ptr[v + 1];
-                    load4(a.sim + (size_t)a.in_src[p0] * a.ld + w0, out);
-                    if (fn == MGV_FN_NOT) {
-#pragma unroll
-                        for (int k = 0; k < SIM_S; ++k) out[k] = ~out[k];
-                    } else if (fn == MGV_FN_MAJ) {
-                        uint64_t b[SIM_S], d[SIM_S];
-                        load4(a.sim + (size_t)a.in_src[p0 + 1] * a.ld + w0, b);
-                        load4(a.sim + (size_t)a.in_src[p0 + 2] * a.ld + w0, d);
-#pragma unroll
-                        for (int k = 0; k < SIM_S; ++k) out[k] = (out[k] & b[k]) | (out[k] & d[k]) | (b[k] & d[k]);
-                    } else {
-                        for (int q = p0 + 1; q < p1; ++q) {
-                            uint64_t b[SIM_S];
-                            load4(a.sim + (size_t)a.in_src[q] * a.ld + w0, b);
-#pragma unroll
-                            for (int k = 0; k < SIM_S; ++k)
-                                out[k] = fn == MGV_FN_AND ? (out[k] & b[k]) : fn == MGV_FN_OR ? (out[k] | b[k]) : (out[k] ^ b[k]);
-                        }
-                    }
+                    gate_words(a, v, fn, w0, out);
                 }
-                uint64_t* dst = a.sim + (size_t)v * a.ld + w0;
-                reinterpret_cast<ulonglong2*>(dst)[0] = make_ulonglong2(out[0], out[1]);
-                reinterpret_cast<ulonglong2*>(dst)[1] = make_ulonglong2(out[2], out[3]);
+                store4(a.sim + (size_t)v * a.ld + w0, out);
                 unsigned cnt = 0;
 #pragma unroll
                 for (int k = 0; k < SIM_S; ++k) cnt += k < nw ? __popcll(out[k]) : 0;
@@ -179,6 +198,131 @@ const char* reason_text(uint32_t why) {
     }
 }
 
+
+// ------------------------------------------------------------------ sequential simulation
+struct SeqArgs {
+    SimArgs s;                      // s.W, s.first_word: the pass's trace words
+    unsigned long long* diff;
+    const int64_t* latches;         // [n_latch][3]: INPUT node, next-state literal, reset
+    const int32_t* slot;            // [N]: latch index of a latch INPUT, -1 elsewhere
+    uint64_t* state;                // [n_latch][ld]
+    const int64_t* pairs;           // [2][P]
+    int32_t n_latch, cycles, warmup;
+    int64_t P, T;
+};
+
+__global__ void __launch_bounds__(SIM_THREADS) seq_sim_kernel(const SeqArgs q) {
+    const SimArgs& a = q.s;
+    const int w0 = blockIdx.x * SIM_S;
+    const int nw = min(SIM_S, a.W - w0);
+    for (int i = threadIdx.x; i < q.n_latch; i += blockDim.x) {           // s_0: the reset state
+        const int64_t r = q.latches[3 * i + 2];
+        uint64_t out[SIM_S];
+        const uint64_t rank = (uint64_t)a.rank[q.latches[3 * i]];
+#pragma unroll
+        for (int k = 0; k < SIM_S; ++k)
+            out[k] = r == 2 ? mix64(a.seed_mixed ^ ((rank << 40) | (uint64_t)(a.first_word + w0 + k))) : r ? ~0ull : 0ull;
+        store4(q.state + (size_t)i * a.ld + w0, out);
+    }
+    __syncthreads();
+    for (int t = 0; t < q.cycles; ++t) {
+        const bool counted = t >= q.warmup;
+        const int64_t gw = (int64_t)t * q.T + a.first_word + w0;
+        for (int l = 0; l < a.L; ++l) {
+            for (int s = 0; s < a.streams; ++s) {
+                const int seg = (s * a.L + l) * MGV_NCODE;
+                const int beg = a.seg_ptr[seg], end = a.seg_ptr[seg + MGV_NCODE];
+                for (int p = beg + threadIdx.x; p < end; p += blockDim.x) {
+                    const int v = a.order[p];
+                    const int fn = node_fn(a, a.code[v]);
+                    uint64_t out[SIM_S] = {0, 0, 0, 0};
+                    if (fn == MGV_FN_INPUT) {
+                        const int j = q.slot[v];
+                        if (j >= 0) {
+                            load4(q.state + (size_t)j * a.ld + w0, out);
+                        } else {
+                            const uint64_t r = (uint64_t)a.rank[v];
+#pragma unroll
+                            for (int k = 0; k < SIM_S; ++k) out[k] = mix64(a.seed_mixed ^ ((r << 40) | (uint64_t)(gw + k)));
+                        }
+                    } else if (fn != MGV_FN_NONE) {
+                        gate_words(a, v, fn, w0, out);
+                    }
+                    store4(a.sim + (size_t)v * a.ld + w0, out);
+                    if (counted) {
+                        unsigned c = 0;
+#pragma unroll
+                        for (int k = 0; k < SIM_S; ++k) c += k < nw ? __popcll(out[k]) : 0;
+                        if (c) atomicAdd(a.ones + v, (unsigned long long)c);
+                    }
+                }
+            }
+            __syncthreads();
+        }
+        if (counted) {
+            for (int64_t p = threadIdx.x; p < q.P; p += blockDim.x) {
+                uint64_t u[SIM_S], w[SIM_S];
+                load4(a.sim + (size_t)q.pairs[p] * a.ld + w0, u);
+                load4(a.sim + (size_t)q.pairs[q.P + p] * a.ld + w0, w);
+                unsigned c = 0;
+#pragma unroll
+                for (int k = 0; k < SIM_S; ++k) c += k < nw ? __popcll(u[k] ^ w[k]) : 0;
+                if (c) atomicAdd(q.diff + p, (unsigned long long)c);
+            }
+        }
+        for (int i = threadIdx.x; i < q.n_latch; i += blockDim.x) {       // s_{t+1}, staged: the walk reads it next cycle
+            const int64_t lit = q.latches[3 * i + 1];
+            uint64_t out[SIM_S];
+            if (lit < 0) {
+#pragma unroll
+                for (int k = 0; k < SIM_S; ++k) out[k] = lit == -1 ? ~0ull : 0ull;
+            } else {
+                load4(a.sim + (size_t)(lit >> 1) * a.ld + w0, out);
+#pragma unroll
+                for (int k = 0; k < SIM_S; ++k) out[k] ^= (lit & 1) ? ~0ull : 0ull;
+            }
+            store4(q.state + (size_t)i * a.ld + w0, out);
+        }
+        __syncthreads();
+    }
+}
+
+// slot[v] = the smallest latch index whose node is v (slot starts at ~0); nodes outside [0, N) are skipped.
+__global__ void latch_slot_kernel(const int64_t* __restrict__ latches, int n_latch, int64_t N, uint32_t* __restrict__ slot) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_latch) return;
+    const int64_t v = latches[3 * i];
+    if (v >= 0 && v < N) atomicMin(slot + v, (uint32_t)i);
+}
+
+enum : uint32_t { BAD_LATCH_NODE = 1, BAD_LATCH_NOT_INPUT, BAD_LATCH_TWICE, BAD_LATCH_NEXT, BAD_LATCH_CIRCUIT, BAD_LATCH_RESET };
+
+// first = min over bad latches of (latch << 8 | reason), starting at ~0.
+__global__ void seq_sim_validate_kernel(const int64_t* __restrict__ latches, int n_latch, int64_t N,
+                                        const int32_t* __restrict__ code, const int32_t* __restrict__ circuit,
+                                        const uint32_t* __restrict__ slot, const SimArgs a,
+                                        unsigned long long* __restrict__ first) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_latch) return;
+    const int64_t v = latches[3 * i], lit = latches[3 * i + 1], r = latches[3 * i + 2];
+    uint32_t why = 0;
+    if (v < 0 || v >= N) why = BAD_LATCH_NODE;
+    else if (node_fn(a, code[v]) != MGV_FN_INPUT) why = BAD_LATCH_NOT_INPUT;
+    else if (slot[v] != (uint32_t)i) why = BAD_LATCH_TWICE;
+    else if (lit < -2 || (lit >> 1) >= N) why = BAD_LATCH_NEXT;
+    else if (lit >= 0 && circuit[lit >> 1] != circuit[v]) why = BAD_LATCH_CIRCUIT;
+    else if (r < 0 || r > 2) why = BAD_LATCH_RESET;
+    if (why) atomicMin(first, ((unsigned long long)i << 8) | why);
+}
+
+int check_cycles(int32_t cycles, int32_t warmup) {
+    MGV_REQUIRE(cycles >= 1, "seq_sim: cycles = %d must be >= 1", cycles);
+    MGV_REQUIRE(warmup >= 0 && warmup < cycles, "seq_sim: warmup = %d must be in [0, cycles = %d)", warmup, cycles);
+    return MGV_OK;
+}
+
+size_t seq_words(int32_t W) { return (size_t)((W > 0 ? W : 0) + SIM_S - 1) / SIM_S * SIM_S; }
+
 }  // namespace
 
 extern "C" size_t mgv_logic_sim_bytes(int64_t N, int32_t W) {
@@ -252,6 +396,120 @@ extern "C" int mgv_logic_sim_pass(const mgv_schedule* sch, const int32_t* code, 
         MGV_CUDA(cudaGetLastError());
         ++launches;
     }
+    mgv_count_launches(launches);
+    return MGV_OK;
+}
+
+extern "C" size_t mgv_seq_sim_bytes(int64_t N, int32_t n_latch, int32_t W) {
+    const size_t n = N > 0 ? (size_t)N : 0;
+    return (n + (n_latch > 0 ? (size_t)n_latch : 0)) * seq_words(W) * sizeof(uint64_t)    // sim rows, state rows
+           + n * sizeof(uint32_t);                                                     // latch slot of every node
+}
+
+extern "C" int mgv_seq_sim_validate(const mgv_schedule* sch, const int32_t* code, const int32_t* fn_table_host,
+                                    const int32_t* circuit, const int64_t* latches, int32_t n_latch, int32_t cycles,
+                                    int32_t warmup, void* ws, size_t ws_bytes, mgv_stream_t stream) {
+    SimArgs a;
+    int rc = fill_args(a, sch, code, fn_table_host);
+    if (rc != MGV_OK) return rc;
+    rc = check_cycles(cycles, warmup);
+    if (rc != MGV_OK) return rc;
+    MGV_REQUIRE(n_latch >= 0 && (n_latch == 0 || (latches && circuit)), "seq_sim_validate: bad latch list");
+    const size_t need = sizeof(unsigned long long) + (size_t)sch->N * sizeof(uint32_t);
+    MGV_REQUIRE(ws && ws_bytes >= need, "seq_sim_validate: workspace < %zu bytes", need);
+    if (n_latch == 0) return MGV_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned long long* first = (unsigned long long*)ws;
+    uint32_t* slot = (uint32_t*)(first + 1);
+    MGV_CUDA(cudaMemsetAsync(ws, 0xff, need, st));
+    const unsigned blocks = (unsigned)((n_latch + 255) / 256);
+    latch_slot_kernel<<<blocks, 256, 0, st>>>(latches, n_latch, sch->N, slot);
+    MGV_CUDA(cudaGetLastError());
+    seq_sim_validate_kernel<<<blocks, 256, 0, st>>>(latches, n_latch, sch->N, code, circuit, slot, a, first);
+    MGV_CUDA(cudaGetLastError());
+    mgv_count_launches(2);
+    unsigned long long host = 0;
+    MGV_CUDA(cudaMemcpyAsync(&host, first, sizeof(host), cudaMemcpyDeviceToHost, st));
+    MGV_CUDA(cudaStreamSynchronize(st));
+    if (host == ~0ull) return MGV_OK;
+    const int i = (int)(host >> 8);
+    int64_t row[3];
+    MGV_CUDA(cudaMemcpy(row, latches + 3 * (size_t)i, sizeof(row), cudaMemcpyDeviceToHost));
+    switch ((uint32_t)(host & 0xff)) {
+        case BAD_LATCH_NODE:
+            mgv_set_error("seq_sim: latch %d: node %lld is outside [0, %d)", i, (long long)row[0], sch->N);
+            break;
+        case BAD_LATCH_NOT_INPUT:
+            mgv_set_error("seq_sim: latch %d: node %lld is not an INPUT", i, (long long)row[0]);
+            break;
+        case BAD_LATCH_TWICE: {
+            uint32_t other = 0;
+            MGV_CUDA(cudaMemcpy(&other, slot + row[0], sizeof(other), cudaMemcpyDeviceToHost));
+            mgv_set_error("seq_sim: latch %d: node %lld appears twice (also latch %u)", i, (long long)row[0], other);
+            break;
+        }
+        case BAD_LATCH_NEXT:
+            mgv_set_error("seq_sim: latch %d: next-state literal %lld names a node outside [0, %d)", i, (long long)row[1],
+                          sch->N);
+            break;
+        case BAD_LATCH_CIRCUIT:
+            mgv_set_error("seq_sim: latch %d: next-state literal %lld names a node of another circuit than node %lld", i,
+                          (long long)row[1], (long long)row[0]);
+            break;
+        default:
+            mgv_set_error("seq_sim: latch %d: reset %lld is not 0, 1 or 2 (uninitialised)", i, (long long)row[2]);
+    }
+    return MGV_ERR_ARG;
+}
+
+extern "C" int mgv_seq_sim_pass(const mgv_schedule* sch, const int32_t* code, const int32_t* input_rank,
+                                const int32_t* fn_table_host, const int64_t* latches, int32_t n_latch, uint64_t seed,
+                                int64_t first_word, int32_t W, int64_t T, int32_t cycles, int32_t warmup, void* ws,
+                                size_t ws_bytes, uint64_t* ones, const int64_t* pairs, int64_t P, uint64_t* diff,
+                                mgv_stream_t stream) {
+    SeqArgs q{};
+    int rc = fill_args(q.s, sch, code, fn_table_host);
+    if (rc != MGV_OK) return rc;
+    rc = check_cycles(cycles, warmup);
+    if (rc != MGV_OK) return rc;
+    MGV_REQUIRE(W > 0 && first_word >= 0 && first_word + W <= T, "seq_sim_pass: W = %d, first_word = %lld, T = %lld", W,
+                (long long)first_word, (long long)T);
+    MGV_REQUIRE((double)cycles * (double)T <= (double)MGV_SEQ_MAX_WORDS, "seq_sim_pass: cycles x T = %d x %lld is above %lld "
+                "input words (a word index would reach the rank bits)", cycles, (long long)T, (long long)MGV_SEQ_MAX_WORDS);
+    MGV_REQUIRE(input_rank && ones, "seq_sim_pass: NULL input_rank or ones");
+    MGV_REQUIRE(n_latch >= 0 && (n_latch == 0 || latches), "seq_sim_pass: bad latch list");
+    MGV_REQUIRE(P >= 0 && (P == 0 || (pairs && diff)), "seq_sim_pass: bad pair list");
+    const size_t need = mgv_seq_sim_bytes(sch->N, n_latch, W);
+    MGV_REQUIRE(ws && ws_bytes >= need && ((uintptr_t)ws & 31) == 0, "seq_sim_pass: workspace < %zu bytes or not 32-byte aligned",
+                need);
+    if (sch->N == 0) return MGV_OK;
+    const size_t ld = seq_words(W), N = (size_t)sch->N;
+    q.s.rank = input_rank;
+    q.s.W = W;
+    q.s.ld = (int)ld;
+    q.s.mode = MGV_SIM_RANDOM;
+    q.s.seed_mixed = mix64(seed);
+    q.s.first_word = first_word;
+    q.s.sim = (uint64_t*)ws;
+    q.s.ones = (unsigned long long*)ones;
+    q.diff = (unsigned long long*)diff;
+    q.latches = latches;
+    q.state = q.s.sim + N * ld;
+    uint32_t* slot = (uint32_t*)(q.state + (size_t)n_latch * ld);
+    q.slot = (const int32_t*)slot;
+    q.pairs = pairs;
+    q.n_latch = n_latch; q.cycles = cycles; q.warmup = warmup;
+    q.P = P; q.T = T;
+    cudaStream_t st = (cudaStream_t)stream;
+    MGV_CUDA(cudaMemsetAsync(slot, 0xff, N * sizeof(uint32_t), st));
+    int launches = 1;
+    if (n_latch > 0) {
+        latch_slot_kernel<<<(unsigned)((n_latch + 255) / 256), 256, 0, st>>>(latches, n_latch, sch->N, slot);
+        MGV_CUDA(cudaGetLastError());
+        ++launches;
+    }
+    seq_sim_kernel<<<(unsigned)(ld / SIM_S), SIM_THREADS, 0, st>>>(q);
+    MGV_CUDA(cudaGetLastError());
     mgv_count_launches(launches);
     return MGV_OK;
 }

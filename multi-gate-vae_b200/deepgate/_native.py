@@ -92,6 +92,10 @@ _PROTOTYPES = {
     "mgv_logic_sim_validate": (ctypes.c_int, [_SP, _vp, _vp, ctypes.POINTER(_i32), _vp, _i64, _vp, _sz, _vp]),
     "mgv_logic_sim_pass": (ctypes.c_int, [_SP, _vp, _vp, ctypes.POINTER(_i32), _i32, ctypes.c_uint64, _i64, _i32,
                                           _vp, _vp, _vp, _i64, _vp, _vp]),
+    "mgv_seq_sim_bytes": (_sz, [_i64, _i32, _i32]),
+    "mgv_seq_sim_validate": (ctypes.c_int, [_SP, _vp, ctypes.POINTER(_i32), _vp, _vp, _i32, _i32, _i32, _vp, _sz, _vp]),
+    "mgv_seq_sim_pass": (ctypes.c_int, [_SP, _vp, _vp, ctypes.POINTER(_i32), _vp, _i32, ctypes.c_uint64, _i64, _i32, _i64,
+                                        _i32, _i32, _vp, _sz, _vp, _vp, _i64, _vp, _vp]),
     "mgv_sim_signature_pass": (ctypes.c_int, [_vp, _i64, _i32, _i64, _vp, _vp, _vp, _vp]),
     "mgv_sim_classes_bytes": (_sz, [_i64]),
     "mgv_sim_classes_group": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _sz, _vp]),

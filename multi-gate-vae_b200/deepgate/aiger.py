@@ -15,10 +15,13 @@ fan-in 2 over distinct predecessors, with no constant node.
     every such use.
   * Constants are folded: AND(x, 0) = 0, AND(x, 1) = x, AND(a, a) = a, AND(a, NOT a) = 0, through the whole graph.  An AND
     that folds to a constant or to another literal is an alias, not a node; an output that folds to a constant gets no node.
-  * Latches are cut: each latch's current-state variable becomes an INPUT node and its next-state literal is treated as an
-    output.  Reset values are read and ignored, so a node fed by a latch is labelled from random (or exhaustive) input
-    patterns like any other input.  Bad-state (B) and constraint (C) literals are outputs too; justice (J) and fairness
-    (F) properties are rejected.  The symbol table and the comment section are skipped.
+  * Latches: each latch's current-state variable becomes an INPUT node and its next-state literal is an output too, so
+    the graph stays combinational.  ``latches`` records the sequential part for ``label_circuits(..., cycles=C)``,
+    which simulates clock cycles from the reset state (deepgate/simulate.py); without ``cycles`` a latch INPUT is
+    labelled from random (or exhaustive) patterns like any other input.  A reset value must be 0, 1 or the latch's own
+    literal (uninitialised), as AIGER 1.9 defines; anything else is an error.  Bad-state (B) and constraint (C) literals
+    are outputs too; justice (J) and fairness (F) properties are rejected.  The symbol table and the comment section
+    are skipped.
 Gate codes come from ``simulate.CODE_TABLES``: ``aig`` INPUT 0, AND 1, NOT 2; ``mig`` / ``xmg`` / ``xag`` INPUT 0, NOT 2,
 AND 3 (an AIG is a valid circuit of each kind, emitted as is).
 
@@ -26,7 +29,9 @@ Besides ``x`` [N, 2] (node id, gate code), ``edge_index`` [E, 2] (src, dst; sort
 file stem), a dict carries ``lit`` int64 [M + 1] and ``outputs`` int64 [O + L + B + C]: the function of every AIGER
 variable and of every output literal (primary outputs, latch next states, bad states, constraints, in file order) as a
 literal over the nodes, ``2 * node + complemented``, where node -1 is the constant 0 (so -2 = 0, -1 = 1).  A variable
-that is neither defined nor used reads -2.  A malformed file raises ``ValueError`` naming the file and the line or byte.
+that is neither defined nor used reads -2.  ``latches`` int64 [L, 3], in file order: the node of the latch's INPUT, its
+next-state literal (the same encoding; equal to ``outputs[O + i]``) and its reset: 0, 1, or 2 for uninitialised.  A
+malformed file raises ``ValueError`` naming the file and the line or byte.
 """
 import os
 
@@ -103,8 +108,8 @@ def _varints(src, buf, base, count):
 
 
 def _parse(src, data):
-    """The netlist as literal arrays: M, O, inputs [I], latches [L, 2] (lhs, next), outputs [O + B + C], ands [A, 3], and
-    ``where(section, index)``, the place of an entry for error messages."""
+    """The netlist as literal arrays: M, O, inputs [I], latches [L, 3] (lhs, next, reset 0 / 1 / 2 = uninitialised),
+    outputs [O + B + C], ands [A, 3], and ``where(section, index)``, the place of an entry for error messages."""
     nl = data.find(b"\n")
     binary, (M, I, L, O, A, B, C) = _header(src, data if nl < 0 else data[:nl])
     n_out = O + B + C
@@ -113,7 +118,7 @@ def _parse(src, data):
         if lines[-1] == b"":
             lines.pop()
         inputs = _rows(src, lines, 1, I, (1,), "input")[:, 0]
-        lat = _rows(src, lines, 1 + I, L, (2, 3), "latch")[:, :2]
+        lat = _rows(src, lines, 1 + I, L, (2, 3), "latch")
         outs = _rows(src, lines, 1 + I + L, n_out, (1,), "output")[:, 0]
         ands = _rows(src, lines, 1 + I + L + n_out, A, (3,), "AND")
         after = 1 + I + L + n_out + A
@@ -129,7 +134,7 @@ def _parse(src, data):
         if rest == b"" and lines[-1] == b"":                     # the newline that ends the file
             lines.pop()
         lat = _rows(src, lines, 1, L, (1, 2), "latch")
-        lat = np.stack([2 * (I + 1 + np.arange(L, dtype=np.int64)), lat[:, 0]], axis=1)
+        lat = np.stack([2 * (I + 1 + np.arange(L, dtype=np.int64)), lat[:, 0], lat[:, 1]], axis=1)
         outs = _rows(src, lines, 1 + L, n_out, (1,), "output")[:, 0]
         inputs = 2 * (1 + np.arange(I, dtype=np.int64))
         base = len(data) - len(rest)                            # file offset of the AND deltas
@@ -149,6 +154,13 @@ def _parse(src, data):
             if section == "and":
                 return "byte %d" % (base + starts[2 * k])
             return "line %d" % (2 + k + (0 if section == "latch" else L))
+    reset = lat[:, 2]                                           # -1: no reset given, which means 0
+    bad = np.flatnonzero((reset > 1) & (reset != lat[:, 0]))
+    if bad.size:
+        k = int(bad[0])
+        raise src.error(where("latch", k), "latch reset %d must be 0, 1 or the latch literal %d (uninitialised)"
+                        % (reset[k], lat[k, 0]))
+    lat = np.stack([lat[:, 0], lat[:, 1], np.where(reset > 1, 2, np.maximum(reset, 0))], axis=1)
     if tail not in (b"", b"\n", b"i", b"l", b"o", b"b", b"c", b"j", b"f"):
         raise src.error(tail_where, "expected the symbol table or the comment section after the %d ANDs the header "
                                     "declares" % A)
@@ -239,8 +251,8 @@ def _fold(M, ands):
 
 def read_aiger(path, kind="aig"):
     """One AIGER file (``.aag`` or ``.aig``, told apart by its header) as a circuit dict with ``x``, ``edge_index``,
-    ``name``, ``lit`` and ``outputs``; the module docstring gives the node order, the folding, the latches and the
-    literal encoding."""
+    ``name``, ``lit``, ``outputs`` and ``latches``; the module docstring gives the node order, the folding, the latches
+    and the literal encoding."""
     if kind not in CODE_TABLES:
         raise ValueError("kind must be one of %s, got %r" % (sorted(CODE_TABLES), kind))
     table = CODE_TABLES[kind]
@@ -278,9 +290,11 @@ def read_aiger(path, kind="aig"):
     e_src = np.concatenate([node[has_not], np.where(fan & 1, not_node[fan >> 1], node[fan >> 1]).reshape(-1)])
     e_dst = np.concatenate([not_node[has_not], np.repeat(start, 2)])
     e = np.lexsort((e_src, e_dst))
+    outputs = 2 * node[out >> 1] + (out & 1)
+    latches = np.stack([node[lat[:, 0] >> 1], outputs[O:O + len(lat)], lat[:, 2]], axis=1).reshape(-1, 3)
     return {"x": np.stack([np.arange(n), gate], axis=1), "edge_index": np.stack([e_src[e], e_dst[e]], axis=1),
             "name": os.path.splitext(os.path.basename(str(path)))[0],
-            "lit": 2 * node[rl >> 1] + (rl & 1), "outputs": 2 * node[out >> 1] + (out & 1)}
+            "lit": 2 * node[rl >> 1] + (rl & 1), "outputs": outputs, "latches": latches.astype(np.int64)}
 
 
 def read_aiger_files(paths, kind="aig"):

@@ -19,10 +19,12 @@ another node's literal.  A node's best cut is its best-ranked cut that matches a
 outputs (of the fan-out-free nodes, for a dict without ``outputs``) and, from the last level down, the leaves of every
 marked node's best cut.  Each marked AND that is not an alias becomes one gate.
 Output dict, in the layout and codes of ``kind``: ``x``, ``edge_index`` [E, 2] sorted by (dst, src), ``name``,
-``outputs`` (each output literal over the new nodes, ``2 node + complemented``; -2 / -1 the constants) and ``origin``
-int64 [N']: the literal over the input circuit's nodes that each new node computes.  Node order: the INPUTs in their
-order, their NOT nodes, then the gates by the id of the AND they replace, each directly followed by its NOT node if it
-has one; one NOT node per complemented node, shared by all of its uses.  Labels of the input are not carried over.
+``outputs`` (each output literal over the new nodes, ``2 node + complemented``; -2 / -1 the constants), ``origin``
+int64 [N']: the literal over the input circuit's nodes that each new node computes, and, when the input has them,
+``latches`` [L, 3] with the latch INPUT nodes and next-state literals over the new nodes (resets as given).  Node
+order: the INPUTs in their order (an AIG whose INPUTs come first, as ``read_aiger`` gives, keeps their ids), their NOT
+nodes, then the gates by the id of the AND they replace, each directly followed by its NOT node if it has one; one NOT
+node per complemented node, shared by all of its uses.  Labels of the input are not carried over.
 """
 import ctypes
 
@@ -260,9 +262,17 @@ def emit(c, kind, arrays):
     e_src = np.concatenate([node[has_not], np.where(use_comp == 1, not_node[use_node], node[use_node])])
     e_dst = np.concatenate([not_node[has_not], node[use_dst]])
     e = np.lexsort((e_src, e_dst))
-    outputs = np.where(rl >= 0, 2 * node[np.maximum(rl, 0) >> 1] + ((rl & 1) ^ out_c[np.maximum(rl, 0) >> 1]), rl)
-    return {"x": np.stack([np.arange(total), gcode], axis=1), "edge_index": np.stack([e_src[e], e_dst[e]], axis=1),
-            "name": c.get("name", ""), "outputs": outputs.astype(np.int64), "origin": origin}
+
+    def new_lit(rl):                                         # final literal -> literal over the new nodes
+        u = np.maximum(rl, 0) >> 1
+        return np.where(rl >= 0, 2 * node[u] + ((rl & 1) ^ out_c[u]), rl).astype(np.int64)
+
+    out = {"x": np.stack([np.arange(total), gcode], axis=1), "edge_index": np.stack([e_src[e], e_dst[e]], axis=1),
+           "name": c.get("name", ""), "outputs": new_lit(rl), "origin": origin}
+    if "latches" in c:                                       # next states are outputs too, so their nodes exist
+        lat = np.asarray(c["latches"], np.int64).reshape(-1, 3)
+        out["latches"] = np.stack([node[lat[:, 0]], new_lit(final(lat[:, 1])), lat[:, 2]], axis=1).reshape(-1, 3)
+    return out
 
 
 def map_circuits(circuits, kind, device, batch_size=64):
